@@ -3,7 +3,7 @@
 bench.py -- ResNet-50 gossip-SGD throughput (BASELINE.json headline metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--algo sgp|osgp|dpsgd|ar]
-                    [--batch-size B] [--impl ours|reference]
+                    [--batch-size B] [--impl ours|reference] [--dump-outputs DIR]
 
 N > 1 is launched by the driver as
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N \
@@ -70,7 +70,16 @@ def parse():
     ap.add_argument('--skip-e2e', action='store_true')
     ap.add_argument('--skip-local', action='store_true',
                     help='skip the gossip-disabled re-measurement behind `exposed_comm` (N > 1)')
-    return ap.parse_args()
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='after the K timed replays behind `value`, write what the last one computed '
+                         '(rank 0) as float32 DIR/<name>.npy: metrics = [loss, prec@1, prec@5], logits, '
+                         'bn_buffers (running statistics) and params (a fixed seeded sample of the '
+                         'updated parameters); inputs are seeded, so two builds can be compared '
+                         'array by array')
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl != 'ours':
+        ap.error('--dump-outputs needs --impl ours')
+    return args
 
 
 # --------------------------------------------------------------------------- #
@@ -180,9 +189,41 @@ def _build(args, dtype, bs, rank, world, dev):
     return net, model, trainer, graph_name
 
 
-def measure(args, dtype, bs, K, W, rank, world, dev, sample_clocks):
+DUMP_MAX_ELEMS = 1 << 22          # per array: 16 MB of float32, so a dump stays well under 64 MB
+
+
+def _dump_sample(flat):
+    """``flat`` itself, or a fixed seeded sample of DUMP_MAX_ELEMS of its elements (sorted indices,
+    the same for every run with the same sizes)."""
+    import numpy as np
+    import torch
+    if flat.numel() <= DUMP_MAX_ELEMS:
+        return flat
+    idx = np.sort(np.random.default_rng(0).choice(flat.numel(), DUMP_MAX_ELEMS, replace=False))
+    return flat.index_select(0, torch.from_numpy(idx).to(flat.device))
+
+
+def dump_outputs(out_dir, net, trainer):
+    """What the last training step handed its caller, as float32 ``out_dir/<name>.npy``."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    logits = trainer.static_out.detach().float()
+    arrays = {
+        'metrics': trainer.static_metrics.detach().float(),          # [loss, prec@1 %, prec@5 %]
+        'logits': logits if logits.numel() <= DUMP_MAX_ELEMS else _dump_sample(logits.reshape(-1)),
+        'bn_buffers': _dump_sample(torch.cat([b.detach().reshape(-1).float() for b in net.buffers()
+                                              if b.is_floating_point()])),
+        'params': _dump_sample(torch.cat([p.detach().reshape(-1).float() for p in net.parameters()])),
+    }
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + '.npy'), t.cpu().numpy().astype(np.float32))
+
+
+def measure(args, dtype, bs, K, W, rank, world, dev, sample_clocks, dump_dir=None):
     """One configuration: W warm-up steps, K device-timed replays (`value`), then K steps through
-    the public API with H2D of the inputs and D2H of [loss, prec@1, prec@5] every step (`e2e`)."""
+    the public API with H2D of the inputs and D2H of [loss, prec@1, prec@5] every step (`e2e`).
+    ``dump_dir``: write what the last of the K timed replays computed there (rank 0)."""
     import torch
     import torch.distributed as dist
     from stochastic_gradient_push_b200.ops import native
@@ -229,6 +270,8 @@ def measure(args, dtype, bs, K, W, rank, world, dev, sample_clocks):
         dist.all_reduce(ms, op=dist.ReduceOp.MAX)
     ms = ms.item()
     value = bs * world * K / (ms / 1e3)
+    if dump_dir and rank == 0:
+        dump_outputs(dump_dir, net, trainer)
 
     # ---- end-to-end timed region (public API, H2D + D2H every step) ---------
     e2e = None
@@ -347,7 +390,8 @@ def run_ours(args):
     torch.backends.cudnn.allow_tf32 = True
 
     bs, K, W = args.batch_size, args.steps, args.warmup
-    main = measure(args, args.dtype, bs, K, W, rank, world, dev, sample_clocks=True)
+    main = measure(args, args.dtype, bs, K, W, rank, world, dev, sample_clocks=True,
+                   dump_dir=args.dump_outputs)
     # secondary, clearly labelled lines: the other precision at the headline batch, and the
     # reference's per-GPU batch (32 images per GPU in its 8-GPU-per-node job scripts), where the
     # gossip step is a larger share of the iteration

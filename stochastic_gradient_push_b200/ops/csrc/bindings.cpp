@@ -175,6 +175,8 @@ public:
         args_.timeout_ns = (unsigned long long)(timeout_s * 1e9);
         keep_.push_back(state);
         keep_.push_back(hyper);
+        c10::cuda::CUDAGuard guard(device_);
+        SGP_CUDA_CHECK(sgp_preload_kernels());      // no first launch may wait for a spinning kernel
         max_grid_ = sgp_max_resident_ctas(device_);
         // the warp-specialised TMA step kernel (default for the full SGP / D-PSGD step) is bound by
         // its dynamic shared memory; the grid has to be co-resident for BOTH kernels because the

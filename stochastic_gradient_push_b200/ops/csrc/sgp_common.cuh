@@ -278,4 +278,5 @@ cudaError_t sgp_launch_barrier(SgpSignalPad* const* pads, SgpState* st, int rank
 cudaError_t sgp_launch_allreduce_sgd(const SgpArgs* args, void* const* grad_peers, int grid,
                                      cudaStream_t stream);
 int sgp_max_resident_ctas(int device);
+cudaError_t sgp_preload_kernels();
 }

@@ -13,6 +13,8 @@
 //   sgp_allreduce_sgd  AR-SGD comparator: one-shot P2P all-reduce fused with SGD
 //   sgp_barrier_kernel device-side barrier over the signal pads
 //   sgp_scale_kernel   flat x *= w  /  x /= w  (ps_numerator / unbias API parity)
+#include <cuda.h>
+
 #include "sgp_common.cuh"
 
 namespace {
@@ -1348,6 +1350,41 @@ int sgp_max_resident_ctas(int device)
     if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, sgp_step_kernel, SGP_THREADS, 0)
         != cudaSuccess) return 0;
     return sms * per_sm;
+}
+
+// With CUDA's lazy loading (the default) a kernel is loaded at its first launch, and that load may
+// have to synchronise the context.  The gossip kernels spin on flags released by other launches: the
+// first launch of sgp_gather_ack_kernel, for instance, is queued while sgp_gather_wait_kernel spins
+// for the in-neighbour, and with several ranks on one host thread (LocalWorld) that in-neighbour's
+// publish is launched only afterwards -- the load would wait for the spin and the spin for the
+// launch, until the heartbeat fires.  Loading every gossip kernel of the current device up front
+// keeps first launches from waiting on the device.
+cudaError_t sgp_preload_kernels()
+{
+    typedef CUresult (*FuncLoad)(CUfunction);
+    static FuncLoad func_load = nullptr;
+    if (func_load == nullptr) {
+        void* p = nullptr;
+        cudaDriverEntryPointQueryResult q;
+        cudaError_t e = cudaGetDriverEntryPoint("cuFuncLoad", &p, cudaEnableDefault, &q);
+        if (e != cudaSuccess) return e;
+        if (q != cudaDriverEntryPointSuccess || p == nullptr) return cudaErrorNotSupported;
+        func_load = reinterpret_cast<FuncLoad>(p);
+    }
+    const void* kernels[] = {
+        (const void*)sgp_step_kernel, (const void*)sgp_step_pipe_kernel, (const void*)sgp_gather_kernel,
+        (const void*)sgp_gather_tma_kernel, (const void*)sgp_probe_kernel, (const void*)sgp_gather_wait_kernel,
+        (const void*)sgp_gather_ack_kernel, (const void*)sgp_bilat_decide_kernel,
+        (const void*)sgp_bilat_ctl_kernel, (const void*)sgp_allreduce_sgd_kernel, (const void*)sgp_zero_kernel,
+        (const void*)sgp_scale_kernel, (const void*)sgp_peer_reduce_kernel, (const void*)sgp_barrier_kernel,
+    };
+    for (const void* k : kernels) {
+        cudaFunction_t f = nullptr;
+        cudaError_t e = cudaGetFuncBySymbol(&f, k);
+        if (e != cudaSuccess) return e;
+        if (func_load(reinterpret_cast<CUfunction>(f)) != CUDA_SUCCESS) return cudaErrorInitializationError;
+    }
+    return cudaSuccess;
 }
 
 }  // extern "C"

@@ -3,6 +3,8 @@ ONE process on ONE GPU (``LocalWorld`` loop-back): the same world-simulation ora
 multi-process tests (tests/test_multigpu.py), but runnable on a single-GPU box -- SGP, D-PSGD,
 Overlap-SGP, the peers_per_itr schedule swap and the graph-captured trainer all exercise the
 flag / ack protocol between kernels that are co-resident on the same device."""
+import gc
+
 import pytest
 import torch
 
@@ -11,6 +13,23 @@ import stochastic_gradient_push_b200 as sgp
 import test_distributed_c10d as sim
 
 pytestmark = pytest.mark.gpu
+
+
+@pytest.fixture(autouse=True)
+def _no_device_sync_from_gc():
+    """One host thread drives every virtual rank, so a rank's gossip kernel can spin until the host
+    launches its in-neighbour's step.  A dropped GossipDataParallel is part of a reference cycle
+    (its hooks hold it) and owns symmetric buffers whose release is a cudaFree, which waits for the
+    whole device: if the cyclic collector freed one between those two launches, the host would
+    wait on a kernel that waits on the host until the heartbeat timeout fired.  So collect while
+    nothing spins, and keep the collector off while the virtual ranks run."""
+    gc.collect()
+    gc.disable()
+    try:
+        yield
+    finally:
+        gc.enable()
+        gc.collect()
 
 
 def _world(n, graph_name, ppi, overlap, fused, nesterov):
@@ -37,8 +56,20 @@ def _world(n, graph_name, ppi, overlap, fused, nesterov):
     return ranks
 
 
+def _load_step_kernels(dev):
+    """Launch the kernels of a training step once before any gossip kernel can spin: a kernel's
+    first launch may load it, and loading may wait for the whole device (the gossip kernels
+    themselves are loaded when their engine is built, see sgp_preload_kernels)."""
+    net = sim._model(0).to(dev)
+    x, y = sim._batch(0, 0)
+    for _ in range(2):          # the second backward accumulates into existing .grad buffers
+        ((net(x.to(dev)) - y.to(dev)) ** 2).mean().backward()
+    torch.cuda.synchronize()
+
+
 def _run(n, graph_name, ppi, steps, overlap, fused, nesterov, ppi_switch=None):
     dev = torch.device('cuda', 0)
+    _load_step_kernels(dev)
     ranks = _world(n, graph_name, ppi, overlap, fused, nesterov)
     for step in range(steps):
         if ppi_switch is not None and step == ppi_switch[0]:
